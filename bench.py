@@ -9,9 +9,13 @@ the grid is (256 N) x 256 and each rank owns one contiguous 256x256 slab (weak s
 section 8e); ``--scaling strong`` splits one 2048x2048 grid over the ranks instead.
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--scaling weak|strong]
+                    [--dump-outputs DIR]
 
 Prints ONE JSON line (rank 0).  ``--impl reference`` times the reference algorithm's CPU path
 (the numpy oracle, all host threads) on a bounded sample of the same workload.
+``--dump-outputs DIR`` writes what the last timed step returned to its caller as DIR/<name>.npy:
+``safe_set`` (float32 0/1 over the global grid) and ``c_max`` (float64, one element).  The inputs
+are seeded, so two builds run with the same arguments can be compared output for output.
 """
 
 from __future__ import annotations
@@ -288,6 +292,11 @@ def run_ours(args, rank, world, local_rank):
     ms_total = max_over_ranks(ms_total)
     value = n_total * args.steps / (ms_total * 1e-3)
     safe_points = int(lyap.last_sweep.get("n_safe", -1))     # first host read-back of the run
+    outputs = None
+    if args.dump_outputs:
+        # what the last timed step hands its caller (reading safe_set is collective over ranks)
+        outputs = {"safe_set": lyap.safe_set.astype(np.float32),
+                   "c_max": np.array([lyap.feed_dict[lyap.c_max]], dtype=np.float64)}
 
     # The timed region lasts K x ~0.3 ms, shorter than one nvidia-smi sample.  The SAME step is
     # therefore continued for ~1.5 s (a fixed count, identical on every rank) under the sampler;
@@ -566,6 +575,10 @@ def run_ours(args, rank, world, local_rank):
         "cpu_baseline": cpu_baseline,
         "safe_points": safe_points, "parity": parity, "exchange": exchange,
     }
+    if outputs is not None:
+        os.makedirs(args.dump_outputs, exist_ok=True)
+        for name, array in outputs.items():
+            np.save(os.path.join(args.dump_outputs, name + ".npy"), array)
     print(json.dumps(line))
     if dist is not None:
         dist.destroy_process_group()
@@ -581,7 +594,11 @@ def main():
                     help="weak: 256x256 per GPU (default); strong: one 2048x2048 grid split over N")
     ap.add_argument("--parity", action="store_true",
                     help="run the oracle parity check even on grids above 2^20 points")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the outputs of the last timed step as DIR/<name>.npy")
     args = ap.parse_args()
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs applies to --impl ours")
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))

@@ -41,6 +41,46 @@ def test_c2_bench_shape_vs_oracle(sl):
     assert_array_equal(gpu.compute_negative().cpu().numpy().astype(bool), det["negative"])
 
 
+def test_bench_dump_outputs_vs_oracle(sl, tmp_path):
+    """`bench.py --dump-outputs DIR` writes what the last timed step handed its caller -- the safe
+    set (float32 0/1) and c_max (float64) -- equal to the oracle's.  Run on the strong-scaling grid
+    (2048 x 2048), where the safe set grows past the initial set, so a dump of the initial mask or
+    of a state before any step would not match.  The launches counted in the timed region are
+    exactly `--steps` sweeps."""
+    import json
+    import os
+    import subprocess
+    import sys
+    import bench
+    from safe_learning_b200 import _native as nat
+    steps = 3
+    out = tmp_path / "outputs"
+    proc = subprocess.run([sys.executable, os.path.join(bench.ROOT, "bench.py"), "--gpus", "1",
+                           "--scaling", "strong", "--steps", str(steps), "--warmup", "0",
+                           "--dump-outputs", str(out)],
+                          stdout=subprocess.PIPE, stderr=subprocess.PIPE, text=True, timeout=900)
+    assert proc.returncode == 0, proc.stderr[-4000:]
+    line = json.loads(proc.stdout.strip().splitlines()[-1])
+    assert sorted(os.listdir(out)) == ["c_max.npy", "safe_set.npy"]
+    safe, c_max = np.load(out / "safe_set.npy"), np.load(out / "c_max.npy")
+    assert safe.dtype == np.float32 and c_max.dtype == np.float64 and c_max.shape == (1,)
+    par = W.make_pendulum(num_points=bench.grid_shape(1, "strong"), M=bench.M_TRAIN,
+                          shared_hypers=False)
+    cpu = W.build_oracle(par)
+    cpu.update_safe_set()                   # stops at the first failing batch: a few seconds
+    assert cpu.safe_set.sum() > par["initial"].sum()
+    assert_array_equal(safe, cpu.safe_set.astype(np.float32))
+    assert c_max[0] == cpu.c_max
+    # launches of one warmed-up sweep (a CUDA-graph replay, like every timed step)
+    gpu = W.build_product(par)
+    for _ in range(3):
+        gpu.update_safe_set()
+    before = nat.launch_count()
+    gpu.update_safe_set()
+    per_sweep = nat.launch_count() - before
+    assert per_sweep > 0 and line["gpu_launches"] == steps * per_sweep
+
+
 def test_c2_bench_shape_growing_safe_set_vs_oracle(sl):
     """Same shape with a finer discretisation constant (tau / 64): 59% of the points satisfy the
     decrease condition, the safe set grows far beyond the initial one and the filter has to hand
